@@ -2,7 +2,7 @@
 """bench.py -- BM25 queries/s of the batched posting-traversal path (BASELINE.json configs[1]):
 10M-doc synthetic Zipf corpus, 1024 three-term disjunctive queries, top-100, on N B200s.
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--workload bm25|conj|knn|hybrid]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--workload bm25|conj|knn|hybrid] [--dump-outputs DIR]
   python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 One "step" = one pass of the hot path over the 1024-query batch. `value` = whole-job queries/s with the compiled batch
@@ -54,7 +54,31 @@ def parse():
     ap.add_argument("--hybrid-dims", type=int, default=128)
     ap.add_argument("--vectors", type=int, default=1_000_000)
     ap.add_argument("--dims", type=int, default=768)
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the results of the last timed step (docs, scores, counts, ...) as DIR/<name>.npy in float32 / float64")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    return args
+
+
+DUMP_LIMIT_BYTES = 60_000_000   # all files together stay below 64 MB, .npy headers included
+
+
+def dump_outputs(out_dir, arrays):
+    """Writes {name: array} with the query as the first axis. Integer arrays become float64 (exact for the doc ids,
+    counts and totals here), float32 stays float32. Above DUMP_LIMIT_BYTES a fixed seeded sample of query rows is written,
+    with their indices as query_rows.npy, so that two builds run with the same arguments write comparable files."""
+    arrays = {name: np.asarray(a, np.float32 if np.asarray(a).dtype == np.float32 else np.float64) for name, a in arrays.items()}
+    nq = len(next(iter(arrays.values())))
+    row_bytes = sum(a.nbytes // nq for a in arrays.values()) + 8
+    if nq * row_bytes > DUMP_LIMIT_BYTES:
+        rows = np.sort(np.random.default_rng(0).choice(nq, DUMP_LIMIT_BYTES // row_bytes, replace=False))
+        arrays = {name: a[rows] for name, a in arrays.items()}
+        arrays["query_rows"] = rows.astype(np.float64)
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
 
 
 def peaks():
@@ -277,10 +301,11 @@ def conj_leg(args, searcher, sh, stream, steps, threads, n_sample):
 
 # ---------------------------------------------------------------------------------------------- kNN (configs[3])
 
-def knn_leg(args, rank, world, local_rank, steps, warmup):
+def knn_leg(args, rank, world, local_rank, steps, warmup, outputs=None):
     """configs[3]: 1M x 768 fp32 vectors, batch-1024 cosine top-100; exact search (tcgen05 bf16 candidate stage, fp64
     re-score, rank-safety certificate). world > 1: the corpus is row-partitioned, every rank searches its shard, ONE
-    all-gather of the packed results, TopDocs.merge on the device."""
+    all-gather of the packed results, TopDocs.merge on the device. `outputs` (a dict) receives the page of the last
+    timed step."""
     import torch
     import oracle
     from nrtsearch_b200 import _native, index as ix
@@ -336,6 +361,8 @@ def knn_leg(args, rank, world, local_rank, steps, warmup):
     wall = (time.perf_counter() - t0) / steps
     sampler.mark_end()
     clocks = sampler.stop() if rank == 0 else None
+    if outputs is not None:
+        outputs.update(docs=out[0].copy(), scores=out[1].copy(), counts=out[2].copy())
     dev_ms = float(np.mean(gemm) + np.mean(sel) + np.mean(resc))
     if world > 1:
         import torch.distributed as dist
@@ -500,7 +527,7 @@ def run_hybrid(args, rank, world, local_rank):
     sampler.mark_begin()
     t0 = time.perf_counter()
     for _ in range(args.steps):
-        step()
+        last = step()
     barrier()
     wall = (time.perf_counter() - t0) / args.steps
     sampler.mark_end()
@@ -523,6 +550,9 @@ def run_hybrid(args, rank, world, local_rank):
             "timing": "host wall clock per step (the step is host-driven: C-ABI calls with host buffers), barrier + synchronize on both sides, max over ranks",
             "gpu_launches": int(stats["launches_per_run"]) + 8, "gate": gate_info, "clocks": clocks,
             "index": {"postings_rank0": int(sh.term_off[-1]), "device_bytes_rank0": gix.device_bytes, "build_s": build_s}}))
+        if args.dump_outputs:
+            (bd, bs, bc, bt), _, _ = last
+            dump_outputs(args.dump_outputs, {"docs": bd, "scores": bs, "counts": bc, "total_hits": bt})
     batch.close(); gix.close(); ctx.close()
     if world > 1:
         dist.destroy_process_group()
@@ -549,7 +579,7 @@ def run_reference(args, rank, world):
     times = []
     for i in range(args.warmup + args.steps):
         t0 = time.perf_counter()
-        oracle.search_compiled(oix, carr, ncl, qarr, nq, args.topk, args.threshold, 1, threads)
+        res = oracle.search_compiled(oix, carr, ncl, qarr, nq, args.topk, args.threshold, 1, threads)
         if i >= args.warmup:
             times.append(time.perf_counter() - t0)
     dt = float(np.mean(times))
@@ -564,6 +594,8 @@ def run_reference(args, rank, world):
         "e2e": {"value": qps, "unit": "queries/s", "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0},
         "note": "restated CPU oracle (oracle/oracle.c, -O3 -march=native), NOT Lucene: no JVM / lucene-core jar exists in this image",
     }))
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, dict(zip(("docs", "scores", "counts", "total_hits", "relation"), res)))
 
 
 # ---------------------------------------------------------------------------------------------- main line
@@ -596,9 +628,12 @@ def main():
         dist.init_process_group("nccl", device_id=torch.device("cuda", local_rank))
     dev = torch.device("cuda", local_rank)
     if args.workload == "knn":
-        line = knn_leg(args, rank, world, local_rank, args.steps, args.warmup)
+        outputs = {}
+        line = knn_leg(args, rank, world, local_rank, args.steps, args.warmup, outputs)
         if rank == 0:
             print(json.dumps(line))
+            if args.dump_outputs:
+                dump_outputs(args.dump_outputs, outputs)
         if world > 1:
             dist.destroy_process_group()
         return
@@ -675,6 +710,9 @@ def main():
     barrier()
     sampler.mark_end()
     clocks = sampler.stop() if rank == 0 else None
+    # the page of the last timed step, read before the e2e leg below reuses pg.local
+    outputs = dict(zip(("docs", "scores", "counts", "relation", "total_hits"), pg.unpack(pg.merged if world > 1 else pg.local))) \
+        if rank == 0 and args.dump_outputs else None
     ms = e0.elapsed_time(e1)
     kernel_ms = batch.stage_ms(0)
     merge_ms = batch.stage_ms(1)
@@ -790,6 +828,8 @@ def main():
             "extra": extra,
         }
         print(json.dumps(line))
+        if outputs:
+            dump_outputs(args.dump_outputs, outputs)
     if ctx is not None:
         ctx.close()
     if world > 1:

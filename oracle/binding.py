@@ -4,6 +4,7 @@ from __future__ import annotations
 import ctypes as C
 import os
 import subprocess
+import tempfile
 
 import numpy as np
 
@@ -47,21 +48,19 @@ def build(force: bool = False) -> str:
     return so
 
 
-def _native_so() -> str:
+def _load_native():
     """liboracle.so rebuilt with -O3 -march=native for the host it runs on (bench.py's cpu_baseline / reference arm: the
     portable build that travels to the GPU box is -march=x86-64-v2). Same sources, same results (-ffp-contract=off, no
-    fast-math); falls back to the portable build when no compiler is present."""
-    so = os.path.join(_HERE, "liboracle_native.so")
-    src = [os.path.join(_HERE, f) for f in ("oracle.c", "oracle.h")]
+    fast-math). It is compiled in a temporary directory, so the source tree may be read-only; returns None (the caller
+    keeps the portable build) when no compiler is present."""
     try:
-        if not os.path.exists(so) or any(os.path.getmtime(x) > os.path.getmtime(so) for x in src):
-            tmp = so + f".{os.getpid()}.tmp"
+        with tempfile.TemporaryDirectory(prefix="nrt_oracle_") as tmp:
+            so = os.path.join(tmp, "liboracle_native.so")
             subprocess.check_call(["gcc", "-O3", "-march=native", "-ffp-contract=off", "-fno-fast-math", "-fPIC", "-fopenmp", "-std=c11",
-                                   "-shared", "-o", tmp, src[0], "-lm"], stderr=subprocess.DEVNULL)
-            os.replace(tmp, so)
-        return so
+                                   "-shared", "-o", so, os.path.join(_HERE, "oracle.c"), "-lm"], stderr=subprocess.DEVNULL)
+            return C.CDLL(so)   # the loaded mapping outlives the file
     except Exception:
-        return ""
+        return None
 
 
 def lib() -> C.CDLL:
@@ -70,9 +69,7 @@ def lib() -> C.CDLL:
         so = os.path.join(_HERE, "liboracle.so")
         if not os.path.exists(so):
             build()
-        if os.environ.get("NRT_ORACLE_NATIVE") == "1":
-            so = _native_so() or so
-        L = C.CDLL(so)
+        L = (_load_native() if os.environ.get("NRT_ORACLE_NATIVE") == "1" else None) or C.CDLL(so)
         L.orc_int_to_byte4.restype = C.c_uint8
         L.orc_int_to_byte4.argtypes = [C.c_int32]
         L.orc_byte4_to_int.restype = C.c_int32
